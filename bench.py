@@ -2,7 +2,7 @@
 """Benchmark of the hot path: input samples/s through the 64-channel gammatone ERB bank.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--strategy slaney]
-                  [--sharding streams|channels] [--distribute]
+                  [--sharding streams|channels] [--distribute] [--dump-outputs DIR]
 
 * A STEP is one pass of the bank over one resident batch of synthetic float32 streams:
   per GPU 4096 streams x 16384 samples (BASELINE.json config 4: "64-channel gammatone ERB
@@ -23,9 +23,13 @@
   timed separately against the NVLink rate. ``--distribute`` (stream sharding): the batch starts
   on rank 0 and is scattered inside the timed region.
 * ``cpu_baseline`` (rank 0, N = 1) and ``--impl reference``: the CPU restatement of the
-  reference's evaluator (oracle/, kind "port": the reference itself is pure Python and lives
-  only in the build container) on the host threads this process may use, median of >= 5
-  repetitions on ONE bounded sample of the same workload.
+  reference's evaluator (oracle/, kind "port": the reference itself is pure Python) on the host
+  threads this process may use, median of 5 repetitions (``--impl reference``: K) on ONE bounded
+  sample of the same workload.
+* ``--dump-outputs DIR`` (GPU run, stream sharding): after the K timed steps, rank 0 writes
+  ``DIR/y.npy``, float32 [n][64][T]: what the last timed step wrote to y[S][64][T] for a fixed,
+  seeded sample of n streams (at most 32 MB; see ``output_sample``).  The inputs are seeded, so
+  two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -43,6 +47,7 @@ UNIT = "input-samples/s"
 S_PER_GPU, T, C, RATE = 4096, 16384, 64, 48000
 BYTES_PER_IN_SAMPLE = 4 + 4 * C     # SURVEY.md section 8(d)
 NVLINK_GBS = 900.0                  # one direction of NVLink 5 per GPU (B200_PROFILING.md)
+DUMP_BYTES = 32 << 20               # --dump-outputs: bytes of y written at most
 
 
 def parse():
@@ -60,7 +65,13 @@ def parse():
   ap.add_argument("--no-e2e", action="store_true")
   ap.add_argument("--no-cpu", action="store_true")
   ap.add_argument("--no-extras", action="store_true", help="skip the secondary records (strategies, cfg2/3/5, generic, stream API)")
-  return ap.parse_args()
+  ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's outputs as DIR/y.npy")
+  args = ap.parse_args()
+  if args.steps < 1:
+    ap.error("--steps must be >= 1")
+  if args.dump_outputs and args.impl == "reference":
+    ap.error("--dump-outputs writes the GPU path's outputs; --impl reference has none")
+  return args
 
 
 def peaks():
@@ -225,7 +236,7 @@ def run_reference(args):
   threads, cpu_info = host_cpus()
   bank = bank_sections(args.strategy)
   port = CpuPort(bank, threads)
-  m = port.measure(max(args.steps, 5), warm=max(args.warmup, 1))
+  m = port.measure(args.steps, warm=max(args.warmup, 1))
   value = m["value"]
   line = {
     "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -264,6 +275,23 @@ class Timer(object):
     e1.record()
     self.barrier()
     return e0.elapsed_time(e1)
+
+
+def output_sample(y):
+  """A fixed, seeded sample of the [S][C][T] float32 device tensor y, as a host array of at most
+  DUMP_BYTES: whole streams (every channel and sample) chosen by numpy default_rng(0), and when one
+  stream alone is larger than that, a sorted seeded sample of its time positions too."""
+  import numpy as np
+  import torch
+  S, Cn, Tn = y.shape
+  rng = np.random.default_rng(0)
+  row_bytes = Cn * Tn * y.element_size()
+  streams = np.sort(rng.choice(S, int(min(S, max(1, DUMP_BYTES // row_bytes))), replace=False))
+  out = y[torch.as_tensor(streams, device=y.device)]
+  if len(streams) * row_bytes > DUMP_BYTES:
+    times = np.sort(rng.choice(Tn, int(DUMP_BYTES // (Cn * y.element_size())), replace=False))
+    out = out[:, :, torch.as_tensor(times, device=y.device)]
+  return out.cpu().numpy()
 
 
 def device_record(torch, dev, plan, S, Tn, steps=5, warm=2, flush=None):
@@ -408,6 +436,8 @@ def run_ours(args):
   local = int(os.environ.get("LOCAL_RANK", "0"))
   if not torch.cuda.is_available():
     raise SystemExit("bench.py needs a GPU (there is no CPU fallback)")
+  if args.dump_outputs and args.sharding == "channels" and world > 1:
+    raise SystemExit("--dump-outputs is not supported with --sharding channels")
   torch.cuda.set_device(local)
   dev = torch.device("cuda", local)
   distributed = world > 1
@@ -471,6 +501,9 @@ def run_ours(args):
   clocks = sampler.stop()
   ms_per_step = ms_total / args.steps
   value = world * S * Tn / (ms_per_step * 1e-3)
+  if args.dump_outputs and rank == 0:        # before anything below launches on y again
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    np.save(os.path.join(args.dump_outputs, "y.npy"), output_sample(y))
 
   # ---- sustained: >= sustain_s of back-to-back launches, own clock record --------------------
   sustained = None

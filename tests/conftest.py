@@ -9,12 +9,10 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
   sys.path.insert(0, ROOT)
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REFERENCE = os.environ.get("ALZ_REFERENCE", "/root/reference")
 
 
 def pytest_configure(config):
   config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-  config.addinivalue_line("markers", "reference: needs the read-only reference checkout (build container only)")
 
 
 def signal(seed, n):
@@ -34,18 +32,15 @@ def vectors():
 
 
 @pytest.fixture(scope="session")
-def reference():
-  """The reference package itself (only in the build container)."""
-  if not os.path.isdir(os.path.join(REFERENCE, "audiolazy")):
-    pytest.skip("reference checkout not present")
-  import warnings
-  sys.dont_write_bytecode = True
-  if REFERENCE not in sys.path:
-    sys.path.append(REFERENCE)
-  with warnings.catch_warnings():
-    warnings.simplefilter("ignore")
-    import audiolazy
-  return audiolazy
+def live():
+  """What the reference computed for tests/test_reference_live.py and test_callers_io.py (make_reference_live.py)."""
+  with open(os.path.join(GOLDEN, "reference_live.json")) as fh:
+    return json.load(fh)
+
+
+@pytest.fixture(scope="session")
+def live_bank():
+  return np.load(os.path.join(GOLDEN, "reference_live_bank.npz"))
 
 
 def rel_err(y, ref):

@@ -1,5 +1,6 @@
 """Callers and data formats either side of the path (SURVEY.md 8f): host-side behaviour on CPU,
-against the live reference where it exists; the filtering itself is covered by the gpu tests."""
+against the reference's outputs stored by tests/golden/make_reference_live.py; the filtering
+itself is covered by the gpu tests."""
 import io
 import struct
 import wave
@@ -40,21 +41,22 @@ def test_wavstream_decoding(bits):
   assert list(ab.WavStream(make_wav(bits, 1, values), keep=True)) == [v + (128 if bits == 8 else 0) for v in values]
 
 
-def test_wavstream_matches_reference(reference):
+def test_wavstream_matches_reference(live):
   values = [0, 100, -100, 32767, -32768, 12345]
-  want = list(reference.WavStream(make_wav(16, 1, values)))
+  want = live["wavstream_16"]
   assert list(ab.WavStream(make_wav(16, 1, values))) == pytest.approx(want, rel=1e-7, abs=1e-9)
 
 
 @pytest.mark.parametrize("bits", [8, 16, 24, 32])
-def test_wavstream_matches_reference_every_width(reference, bits):
+def test_wavstream_matches_reference_every_width(live, bits):
   """Byte formats must be bit-exact: same floats (and same ints with keep=True) as the reference's WavStream."""
   top = 1 << (bits - 1)
   values = [0, 1, -1, top - 1, -top, top // 3, -(top // 7), 12345 % top, -(54321 % top)]
   for channels in (1, 2):
     vals = values if channels == 1 else values + values[::-1]
-    assert list(ab.WavStream(make_wav(bits, channels, vals))) == list(reference.WavStream(make_wav(bits, channels, vals)))
-    assert list(ab.WavStream(make_wav(bits, channels, vals), keep=True)) == list(reference.WavStream(make_wav(bits, channels, vals), keep=True))
+    want = live["wavstream_widths"][str(bits)][str(channels)]
+    assert list(ab.WavStream(make_wav(bits, channels, vals))) == want["float"]
+    assert list(ab.WavStream(make_wav(bits, channels, vals), keep=True)) == want["keep"]
 
 
 def test_chunks():
@@ -66,10 +68,10 @@ def test_chunks():
   assert list(ab.chunks([])) == []
 
 
-def test_chunks_match_reference(reference):
+def test_chunks_match_reference(live):
   data = [0.5, -0.25, 1.0, 0.125, -1.0]
-  assert list(ab.chunks(data, size=4)) == list(reference.chunks(data, size=4))
-  assert list(ab.chunks(data, size=2, dfmt="d", padval=9.)) == list(reference.chunks(data, size=2, dfmt="d", padval=9.))
+  assert list(ab.chunks(data, size=4)) == [bytes.fromhex(h) for h in live["chunks_f4"]]
+  assert list(ab.chunks(data, size=2, dfmt="d", padval=9.)) == [bytes.fromhex(h) for h in live["chunks_d2_pad9"]]
 
 
 def test_wav_batch(tmp_path):
@@ -95,11 +97,10 @@ def test_sources_and_maverage_designs():
   assert ab.accumulate_z.denlist == [1, -1]
 
 
-def test_designs_match_reference(reference):
+def test_designs_match_reference(live):
   for size in (1, 3, 8):
     for name in ("recursive", "fir"):
-      mine, theirs = ab.maverage[name](size), reference.maverage[name](size)
-      assert mine.numlist == list(theirs.numlist) and mine.denlist == list(theirs.denlist)
+      mine, theirs = ab.maverage[name](size), live["maverage"]["%s_%d" % (name, size)]
+      assert [mine.numlist, mine.denlist] == theirs
   ks = ab.comb.tau(2 * np.pi / 0.05, 2e4).linearize()
-  kr = reference.comb.tau(2 * np.pi / 0.05, 2e4).linearize()
-  assert ks.numlist == list(kr.numlist) and ks.denlist == list(kr.denlist)
+  assert [ks.numlist, ks.denlist] == live["comb_tau_linearized"]
